@@ -60,7 +60,35 @@ def parse():
     ap.add_argument('--workload', default='c2', choices=sorted(WORKLOADS))
     ap.add_argument('--inflight', type=int, default=3,
                     help='scans in flight per GPU in the timed legs (harness.ScanPipeline); 1 = strictly one after another')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the result of the last timed device step (rank 0) as DIR/<name>.npy, for comparing builds')
     return ap.parse_args()
+
+
+DUMP_BUDGET = 64 << 20
+
+
+def dump_outputs(out, path):
+    """The arrays of a forward_test(device_only=True) result as float32 (floating point) or float64 (integers and masks,
+    exact) .npy files. Above DUMP_BUDGET bytes in all, every array keeps a fixed, seeded sample of its rows."""
+    flat = dict(out.get('device_instances') or {})
+    flat = {'instance_' + k: v for k, v in flat.items()}
+    for k in ('semantic_preds', 'pt_offsets', 'proposals_idx', 'proposals_offset'):
+        flat[k] = out[k]
+    arrs = {}
+    for k, v in flat.items():
+        a = v.detach().cpu().numpy()
+        arrs[k] = a.astype(np.float32 if np.issubdtype(a.dtype, np.floating) else np.float64)
+    total = sum(a.nbytes for a in arrs.values())
+    if total > DUMP_BUDGET:
+        frac = DUMP_BUDGET / float(total)
+        for k, a in arrs.items():
+            n = a.shape[0]
+            rows = np.sort(np.random.RandomState(0).permutation(n)[:int(n * frac)])
+            arrs[k] = a[rows]
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(path, k + '.npy'), a)
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -539,6 +567,8 @@ def main():
         seq_dev_ms, dev_wall, out = timed(step_device, args.steps, max(args.warmup, 3))
         launches = (_lib.lib().sgb_launch_count() - l0)
         seq_dev_steps = sorted(timed.last_per_step)
+        if args.dump_outputs and rank == 0:  # before the later legs run the model on this thread again
+            dump_outputs(out, args.dump_outputs)
         seq_e2e_ms, e2e_wall, ret = timed(lambda: harness.run_scan(model, hb, inject_pointwise=inj), args.steps, 3)
         seq_e2e_steps = sorted(timed.last_per_step)
         if pipe is not None:

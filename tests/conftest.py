@@ -33,35 +33,17 @@ def golden():
 
 
 @pytest.fixture(scope='session')
-def ref_ops():
-    """The compiled, unmodified reference extension (oracle/_ref) or None."""
-    from oracle.build_ref import load_ref
-    try:
-        return load_ref()
-    except Exception:
-        return None
+def host_gold():
+    """What the original project's host code returned on the tests' inputs (tests/golden/make_reference_golden.py)."""
+    import json
+    with open(os.path.join(ROOT, 'tests', 'golden', 'ref_host.json')) as f:
+        return json.load(f)
 
 
 @pytest.fixture(scope='session')
-def ref_model_module():
-    """The UNMODIFIED reference `softgroup/model/softgroup.py`, imported on top of this repo's spconv / ops shims
-    (build container only; None where /root/reference is absent)."""
-    ref_root = '/root/reference'
-    if not os.path.isdir(ref_root):
-        return None
-    import importlib
-    import types
-    import softgroup_b200
-    softgroup_b200.install_as_reference_backends()
-    pkg = types.ModuleType('softgroup')
-    pkg.__path__ = [os.path.join(ref_root, 'softgroup')]
-    sys.modules.setdefault('softgroup', pkg)
-    util = types.ModuleType('softgroup.util')
-    from softgroup_b200 import util as our_util
-    for n in ('cuda_cast', 'force_fp32', 'rle_decode', 'rle_encode'):
-        setattr(util, n, getattr(our_util, n))
-    sys.modules.setdefault('softgroup.util', util)
-    return importlib.import_module('softgroup.model.softgroup')
+def host_arrays():
+    import numpy as np
+    return np.load(os.path.join(ROOT, 'tests', 'golden', 'ref_host.npz'))
 
 
 @pytest.fixture

@@ -256,34 +256,25 @@ def test_clusters_voxelization_equals_reference_steps(monkeypatch):
 
 
 # ---- the reference's OWN forward_grouping (unmodified class on our shims) as the golden -------------------------
-def test_forward_grouping_equals_reference_method(monkeypatch, ref_model_module):
-    """softgroup/model/softgroup.py:411-480 itself runs on CPU once its three CUDA touch points (ball_query,
-    bfs_cluster, get_batch_offsets' .cuda()) are replaced by oracle stand-ins; ours must return the same tensors."""
-    if ref_model_module is None:
-        pytest.skip('reference tree not mounted')
-    import types
+def forward_grouping_inputs():
+    """(semantic scores, offsets, batch_idxs, coords_float) of a 2000-point scan."""
+    sc = synth.make_scan('c1_plumbing', seed=7, n_points=2000)
+    scores, offs = synth.grouping_inputs(sc, sigma=0.03, seed=7)
+    return [torch.from_numpy(scores), torch.from_numpy(offs), torch.zeros(scores.shape[0], dtype=torch.int32),
+            torch.from_numpy(sc['coords_float'])]
+
+
+def test_forward_grouping_equals_reference_method(monkeypatch, host_arrays):
+    """softgroup/model/softgroup.py:411-480 itself ran on CPU once its three CUDA touch points (ball_query, bfs_cluster,
+    get_batch_offsets' .cuda()) were replaced by oracle stand-ins (tests/golden/make_reference_golden.py); ours must
+    return the same tensors."""
     cfg = model_cfg('scannet', channels=16, num_blocks=2, test_cfg=dict(min_npoint=30))
     ours = SoftGroup(**cfg).eval()
-    ref = ref_model_module.SoftGroup(**cfg)
-    ref.eval()
-    ref.test_cfg = types.SimpleNamespace(**cfg['test_cfg'])
-    ref.grouping_cfg = types.SimpleNamespace(**cfg['grouping_cfg'])
-    ref.get_batch_offsets = ours.get_batch_offsets
-
-    def ref_bfs(mean, idxs, start_len, thr, class_id):
-        a, b = oracle.bfs_cluster(mean.numpy(), idxs.numpy(), start_len.numpy(), thr, class_id)
-        return torch.from_numpy(a.astype(np.int32)), torch.from_numpy(b.astype(np.int32))
-
-    monkeypatch.setattr(ref_model_module, 'ball_query', _fake_ball_query)
-    monkeypatch.setattr(ref_model_module, 'bfs_cluster', ref_bfs)
     monkeypatch.setattr(sg_module, 'ballquery_batch_p_nosync', _fake_ballquery_nosync)
     monkeypatch.setattr(sg_module, 'bfs_cluster_segments', _fake_bfs_segments)
     monkeypatch.setattr(sg_module, 'group_entries', _fake_group_entries)
-    sc = synth.make_scan('c1_plumbing', seed=7, n_points=2000)
-    scores, offs = synth.grouping_inputs(sc, sigma=0.03, seed=7)
-    args = [torch.from_numpy(scores), torch.from_numpy(offs), torch.zeros(scores.shape[0], dtype=torch.int32),
-            torch.from_numpy(sc['coords_float'])]
-    want_idx, want_off = ref.forward_grouping(*[a.clone() for a in args], ref.grouping_cfg)
-    got_idx, got_off = ours.forward_grouping(*[a.clone() for a in args])
+    want_idx = torch.from_numpy(host_arrays['forward_grouping_idx'])
+    want_off = torch.from_numpy(host_arrays['forward_grouping_off'])
+    got_idx, got_off = ours.forward_grouping(*forward_grouping_inputs())
     assert want_off.numel() > 2
-    assert torch.equal(got_idx, want_idx.int()) and torch.equal(got_off, want_off.int())
+    assert torch.equal(got_idx, want_idx) and torch.equal(got_off, want_off)

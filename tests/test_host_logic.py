@@ -1,7 +1,5 @@
 """Host-side logic that needs no GPU: weight packing layout, RLE wire format (numpy path and the library's host
 formatter), config values against the reference YAMLs, BatchNorm folding, synthetic-scan layout."""
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -9,9 +7,6 @@ import torch
 from softgroup_b200 import configs, synth
 from softgroup_b200.spconv import core
 from softgroup_b200.util import rle as rle_util
-
-REF = '/root/reference'
-
 
 # ---- tcgen05 weight packing (include/sgb200.h: Wp fp16 [K][nkc][4][2][N][8]) ------------------------------------
 @pytest.mark.parametrize('K,Cin,Cout', [(1, 6, 32), (3, 40, 20), (8, 32, 64), (27, 96, 96)])
@@ -80,16 +75,17 @@ def test_rle_encode_many_empty():
     assert rle_util.rle_encode_many(np.zeros(0, np.int32), np.zeros(1, np.int64), 10) == []
 
 
-# ---- configs are restated data: pin them on the reference YAMLs where the reference tree is present -------------
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree not mounted (GPU box)')
-@pytest.mark.parametrize('name,path', [('scannet', 'configs/softgroup/softgroup_scannet.yaml'),
-                                       ('s3dis', 'configs/softgroup/softgroup_s3dis_fold5.yaml'),
-                                       ('kitti', 'configs/softgroup/softgroup_kitti.yaml'),
-                                       ('stpls3d++', 'configs/softgroup++/softgroup++_stpls3d.yaml'),
-                                       ('scannet++', 'configs/softgroup++/softgroup++_scannet.yaml')])
-def test_configs_match_reference_yaml(name, path):
-    import yaml
-    ref = yaml.safe_load(open(os.path.join(REF, path)))['model']
+# ---- configs are restated data: pinned on the `model` sections of the reference YAMLs (tests/golden/ref_host.json) -----
+CONFIG_FILES = [('scannet', 'configs/softgroup/softgroup_scannet.yaml'),
+                ('s3dis', 'configs/softgroup/softgroup_s3dis_fold5.yaml'),
+                ('kitti', 'configs/softgroup/softgroup_kitti.yaml'),
+                ('stpls3d++', 'configs/softgroup++/softgroup++_stpls3d.yaml'),
+                ('scannet++', 'configs/softgroup++/softgroup++_scannet.yaml')]
+
+
+@pytest.mark.parametrize('name,path', CONFIG_FILES)
+def test_configs_match_reference_yaml(host_gold, name, path):
+    ref = host_gold['configs'][name]
     ours = configs.model_cfg(name)
     for key in ('channels', 'num_blocks', 'semantic_classes', 'instance_classes', 'sem2ins_classes', 'semantic_only',
                 'ignore_label'):

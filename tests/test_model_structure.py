@@ -1,16 +1,10 @@
-"""CPU: the module tree / state_dict contract. When the reference tree is present (build container only),
-the UNMODIFIED reference SoftGroup class is instantiated on top of this repo's spconv/ops shims and its
-state_dict keys and shapes must equal ours one to one (checkpoints load unchanged, softgroup/util/utils.py:111-145)."""
-import os
-import sys
-
-import pytest
+"""CPU: the module tree / state_dict contract. The state_dict keys and shapes of the UNMODIFIED reference SoftGroup class
+(instantiated on this repo's spconv/ops shims; tests/golden/ref_host.json) must equal ours one to one (checkpoints load
+unchanged, softgroup/util/utils.py:111-145)."""
 import torch
 
 from softgroup_b200.configs import model_cfg
 from softgroup_b200.model import SoftGroup
-
-REF = '/root/reference'
 
 
 def test_state_dict_names():
@@ -29,30 +23,14 @@ def test_state_dict_names():
     assert n_subm == 53 + 12  # backbone + tiny U-Net
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree only exists in the build container')
-def test_reference_class_on_our_shims_has_identical_state_dict():
-    import importlib
-    import types
-    import softgroup_b200
-    softgroup_b200.install_as_reference_backends()
-    # load the reference's model package without importing softgroup/__init__ side effects
-    pkg = types.ModuleType('softgroup')
-    pkg.__path__ = [os.path.join(REF, 'softgroup')]
-    sys.modules.setdefault('softgroup', pkg)
-    util = types.ModuleType('softgroup.util')
-    from softgroup_b200 import util as our_util
-    for n in ('cuda_cast', 'force_fp32', 'rle_decode', 'rle_encode'):
-        setattr(util, n, getattr(our_util, n))
-    sys.modules.setdefault('softgroup.util', util)
-    ref_model = importlib.import_module('softgroup.model.softgroup')
-    cfg = model_cfg('scannet')
-    ref = ref_model.SoftGroup(**cfg)
-    ours = SoftGroup(**cfg)
-    a, b = ref.state_dict(), ours.state_dict()
-    assert list(a.keys()) == list(b.keys())
-    for k in a:
-        assert a[k].shape == b[k].shape, k
-    ours.load_state_dict(a)  # strict
+def test_reference_class_on_our_shims_has_identical_state_dict(host_gold):
+    want = host_gold['state_dict']
+    ours = SoftGroup(**model_cfg('scannet'))
+    b = ours.state_dict()
+    assert [k for k, _ in want] == list(b.keys())
+    for k, shape in want:
+        assert list(b[k].shape) == shape, k
+    ours.load_state_dict({k: torch.zeros(shape, dtype=b[k].dtype) for k, shape in want})  # strict
 
 
 def test_model_survives_deepcopy_and_pickle():

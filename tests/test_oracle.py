@@ -1,11 +1,19 @@
-"""CPU: the oracle (oracle/sg_oracle.c) against the golden vectors produced by the compiled reference,
-and, where the reference extension is present (oracle/_ref), against the reference itself on fresh inputs."""
+"""CPU: the oracle (oracle/sg_oracle.c) against the golden vectors produced by the compiled reference, and against what
+the compiled reference returned on the fresh inputs built below (tests/golden/ref_host.json, digests;
+tests/golden/make_reference_golden.py)."""
+import os
+import sys
+
 import numpy as np
 import pytest
-import torch
 
 import oracle
 from softgroup_b200 import synth
+
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden'))
+from digest import digest  # noqa: E402
+
+FRESH_BFS_THRESHOLDS = [(0.5, 5), (2.0, 5), (3.0, 0)]
 
 
 def test_voxelize_idx_golden_c1(golden):
@@ -65,63 +73,59 @@ def test_ballquery_cap():
     assert np.array_equal(idx[:1000], np.arange(1000))
 
 
-def test_vs_reference_fresh(ref_ops):
-    if ref_ops is None:
-        pytest.skip('oracle/_ref not built')
+def fresh_inputs():
+    """A hashed scan and random asymmetric graphs incl. duplicates inside a list: (coords, class means, [(n, idx, sl)])."""
     scan = synth.make_scan('c1_plumbing', seed=3, n_points=5000)
-    c = torch.from_numpy(scan['coords'])
-    oc, im, om = c.new(), torch.IntTensor(c.size(0)).zero_(), torch.IntTensor()
-    ref_ops.voxelize_idx(c, oc, im, om, 1, 4)
-    a, b, d = oracle.voxelization_idx(scan['coords'], 1, 4)
-    assert np.array_equal(a, oc.numpy()) and np.array_equal(b, im.numpy()) and np.array_equal(d, om.numpy())
-    # bfs on random asymmetric graphs incl. duplicates inside a list
     rng = np.random.RandomState(5)
     mean = np.full(20, -1, np.float32)
+    graphs = []
     for t in range(20):
         n = rng.randint(5, 120)
         lens = rng.randint(0, 6, n)
         idx = rng.randint(0, n, int(lens.sum()) + 1).astype(np.int32)
         sl = np.stack([np.concatenate([[0], np.cumsum(lens)[:-1]]), lens], 1).astype(np.int32)
-        ci, co = torch.IntTensor(), torch.IntTensor()
-        ref_ops.bfs_cluster(torch.from_numpy(mean), torch.from_numpy(idx), torch.from_numpy(sl), ci, co, n, 2.0, 0)
-        oi, oo = oracle.bfs_cluster(mean, idx, sl, 2.0, 0)
-        assert np.array_equal(oi, ci.numpy().reshape(-1, 2)) and np.array_equal(oo, co.numpy())
+        graphs.append((n, idx, sl))
+    return scan['coords'], mean, graphs
 
 
-@pytest.mark.parametrize('seed', range(4))
-def test_vs_reference_fresh_more(ref_ops, seed):
-    """More fresh-input comparisons with the compiled reference: batched hashing with duplicates and empty batches,
-    class-mean (relative) BFS thresholds, octree build on clustered points."""
-    if ref_ops is None:
-        pytest.skip('oracle/_ref not built')
+def fresh_more_inputs(seed):
+    """-> (batched coords, (points, ball-query lists, start_len, class means), clustered cloud for the octree)."""
     rng = np.random.RandomState(100 + seed)
-    # voxelize_idx: 3 batch items (one empty), heavy duplication, every mode
+    # voxelize_idx: 3 batch items (one empty), heavy duplication
     n = 4000
     b = rng.choice([0, 2], n)  # batch item 1 stays empty
     xyz = rng.randint(0, 12, (n, 3))
     coords = np.concatenate([b[:, None], xyz], 1).astype(np.int64)
     coords = coords[np.argsort(b, kind='stable')]
-    for mode in (1, 2, 3, 4):
-        c = torch.from_numpy(coords)
-        oc, im, om = c.new(), torch.IntTensor(c.size(0)).zero_(), torch.IntTensor()
-        ref_ops.voxelize_idx(c, oc, im, om, 3, mode)
-        a, bb, d = oracle.voxelization_idx(coords, 3, mode)
-        assert np.array_equal(a, oc.numpy()) and np.array_equal(bb, im.numpy()) and np.array_equal(d, om.numpy()), mode
-    # bfs_cluster with relative thresholds (threshold * class mean, bfs_cluster.cpp:70-77) on ball-query graphs
     pts = (rng.rand(700, 3) * np.array([1.0, 1.0, 0.3])).astype(np.float32)
     idx, sl = oracle.ballquery_batch_p(pts, np.zeros(700, np.int32), np.array([0, 700], np.int32), 0.09)
     mean = np.full(20, -1, np.float32)
     mean[5] = 40.0
-    for thr, cls in [(0.5, 5), (2.0, 5), (3.0, 0)]:
-        ci, co = torch.IntTensor(), torch.IntTensor()
-        ref_ops.bfs_cluster(torch.from_numpy(mean), torch.from_numpy(idx), torch.from_numpy(sl), ci, co, 700, thr, cls)
-        oi, oo = oracle.bfs_cluster(mean, idx, sl, thr, cls)
-        assert np.array_equal(oi, ci.numpy().reshape(-1, 2)) and np.array_equal(oo, co.numpy()), (thr, cls)
-    # octree build (octree_ball_query.cpp:19-165)
     cl = (rng.randn(3000, 3) * 0.2 + rng.randint(0, 4, (3000, 1))).astype(np.float32)
-    boxes, pt_inds, psl = oracle.build_octree(cl)
-    rb, rp, rs = torch.zeros(585, 6), torch.zeros(3000, dtype=torch.int32), torch.zeros(512, 2, dtype=torch.int32)
-    mx, mn = cl.max(0), cl.min(0)  # the Python wrapper passes (centre, extent) of the cloud (functions.py:19-24)
-    xyzwhl = torch.from_numpy(np.concatenate([(mx + mn) / np.float32(2), mx - mn]).astype(np.float32))
-    ref_ops.build_and_export_octree(torch.from_numpy(cl), xyzwhl, rb, rp, rs, 3)
-    assert np.array_equal(boxes, rb.numpy()) and np.array_equal(pt_inds, rp.numpy()) and np.array_equal(psl, rs.numpy())
+    return coords, (pts, idx, sl, mean), cl
+
+
+def _digests(arrays):
+    return [digest(a) for a in arrays]
+
+
+def test_vs_reference_fresh(host_gold):
+    coords, mean, graphs = fresh_inputs()
+    assert _digests(oracle.voxelization_idx(coords, 1, 4)) == host_gold['fresh_vox']
+    for (n, idx, sl), want in zip(graphs, host_gold['fresh_bfs']):
+        assert _digests(oracle.bfs_cluster(mean, idx, sl, 2.0, 0)) == want
+    assert len(graphs) == len(host_gold['fresh_bfs'])
+
+
+@pytest.mark.parametrize('seed', range(4))
+def test_vs_reference_fresh_more(host_gold, seed):
+    """More fresh-input comparisons with the compiled reference: batched hashing with duplicates and empty batches,
+    class-mean (relative) BFS thresholds, octree build on clustered points."""
+    coords, (pts, idx, sl, mean), cl = fresh_more_inputs(seed)
+    for mode, want in zip((1, 2, 3, 4), host_gold['more%d_vox' % seed]):
+        assert _digests(oracle.voxelization_idx(coords, 3, mode)) == want, mode
+    # bfs_cluster with relative thresholds (threshold * class mean, bfs_cluster.cpp:70-77) on ball-query graphs
+    for (thr, cls), want in zip(FRESH_BFS_THRESHOLDS, host_gold['more%d_bfs' % seed]):
+        assert _digests(oracle.bfs_cluster(mean, idx, sl, thr, cls)) == want, (thr, cls)
+    # octree build (octree_ball_query.cpp:19-165)
+    assert _digests(oracle.build_octree(cl)) == host_gold['more%d_octree' % seed]
